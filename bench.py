@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — fwd+bwd views/s of the rasterizer hot path on synthetic 1080p / 3M-Gaussian / SH-3 scenes.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-cpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-cpu] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one view: rasterize() forward + backward of the image
@@ -22,6 +22,10 @@ ONE JSON line (contract: see the round prompt / DESIGN.md "Measurement").
                       reference's own CUDA rasterizer" target is defined against.  The reference has no CPU
                       implementation of this path; when oracle/_ref is absent this falls back to
 --impl reference-cpu  the CPU oracle port on the host cores (bounded sample).
+
+--dump-outputs DIR    (b200) after the timed resident steps, write what the last of them computed to DIR/<name>.npy
+                      (see dump_outputs); the inputs depend only on the arguments, so two builds run with the same
+                      arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -45,6 +49,7 @@ N_GAUSS = 3_000_000
 RES = "1080p"
 SH_DEGREE = 3
 N_POSES = 8
+DUMP_ROWS = 65_536  # gaussians whose per-gaussian outputs --dump-outputs writes (fixed seeded sample of N_GAUSS)
 MY_KERNELS = ["k_camera_centre", "k_preprocess_fwd", "k_emit_pairs_fused", "k_tile_ranges", "k_render_fwd",
               "k_render_bwd", "k_preprocess_bwd"]  # + k_gather_records_keys with GSR_RECORD_STREAM=1
 
@@ -200,6 +205,29 @@ def timed_steps(step_fn, steps, warmup, world, dev):
 _LAST_PER_RANK_MS = []  # ms of the last timed_steps() call on every rank (explains max-over-ranks at N > 1)
 
 
+def dump_outputs(out_dir, image, mask, uv, g):
+    """What one step returned to its caller, as float32 / float64 .npy files (about 41 MB): the image in full and, for
+    a fixed seeded sample of DUMP_ROWS gaussians (gaussian_rows), the culling mask (1 = culled), uv (0 where
+    culled: a culled gaussian has no projection) and the gradient of every parameter.  Every value is finite."""
+    import numpy as np
+    import torch
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    n = g.xyz.shape[0]
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    at = rows.to(mask.device)
+    uv_all = torch.zeros((n, 2), device=uv.device)
+    uv_all[~mask] = uv.detach()
+    arrays = {"image": image.detach(), "gaussian_rows": rows.double(), "culling_mask": mask[at].float(),
+              "uv": uv_all[at]}
+    for name in ("xyz", "rgb", "opacity", "scale", "quaternion", "sh"):
+        arrays["grad_" + name] = getattr(g, name).grad[at]
+    for name, t in arrays.items():
+        np.save(out / f"{name}.npy", t.cpu().numpy())
+    return sorted(arrays)
+
+
 def run_b200(args, rank, world, local):
     import torch
 
@@ -220,11 +248,15 @@ def run_b200(args, rank, world, local):
         # pinned to the heaviest view (P differs by ~1.5% between poses) when the max over ranks is taken
         return (i + rank) % N_POSES
 
+    last = {}  # the outputs of the latest resident step, kept only for --dump-outputs
+
     def step_resident(i):
         zero_grads(g)
-        image, _, _ = rasterize(g, poses[view_of(i)], cam, cfg["near_thresh"], cfg["far_thresh"],
-                                cfg["cull_mask_padding"], cfg["mh_dist"], True, bg)
+        image, mask, uv = rasterize(g, poses[view_of(i)], cam, cfg["near_thresh"], cfg["far_thresh"],
+                                    cfg["cull_mask_padding"], cfg["mh_dist"], True, bg)
         image.backward(G)
+        if args.dump_outputs:
+            last.update(image=image, mask=mask, uv=uv)
 
     h2d_bytes = poses_host[0].numel() * 4 + K_host.numel() * 4 + G_host.numel() * 4
     d2h_bytes = image_host.numel() * 4
@@ -264,6 +296,11 @@ def run_b200(args, rank, world, local):
     log("timing: resident")
     ms_res = timed_steps(step_resident, args.steps, args.warmup, world, dev)
     per_rank_res = [m / args.steps for m in _LAST_PER_RANK_MS]
+    if args.dump_outputs and rank == 0:  # the gradients of the last resident step are still on the parameters
+        names = dump_outputs(args.dump_outputs, last["image"], last["mask"], last["uv"], g)
+        log(f"outputs of step {args.warmup + args.steps - 1} (view {view_of(args.warmup + args.steps - 1)}) written "
+            f"to {args.dump_outputs}: {', '.join(names)}")
+    last.clear()
     log(f"resident {ms_res / args.steps:.3f} ms/step; timing: e2e")
     ms_e2e = timed_steps(step_e2e, args.steps, args.warmup, world, dev)
     per_rank_e2e = [m / args.steps for m in _LAST_PER_RANK_MS]
@@ -595,7 +632,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "reference-cpu", "cpu-baseline-child"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed resident step computed to DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     rank, world, local = dist_env()
     if args.impl == "cpu-baseline-child":  # internal: the sandboxed CPU leg (see cpu_baseline_sandboxed)

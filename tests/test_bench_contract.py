@@ -91,3 +91,43 @@ def test_every_arm_names_the_same_workload():
     src = (ROOT / "bench.py").read_text()
     assert src.count('"workload": WORKLOAD') == 3 and bench.WORKLOAD.startswith("synthetic 3M Gaussians, 1080p, SH deg 3")
     assert bench.METRIC.startswith("fwd+bwd views/sec @1080p, 3M Gaussians")
+
+
+def test_dumped_outputs_are_finite_float_arrays_within_64_mb(tmp_path):
+    """--dump-outputs writes float32 / float64 arrays, all finite (culled gaussians included), at most 64 MB in all
+    at the bench's image size and sample size; the sample of gaussians is the same from run to run."""
+    import importlib.util
+
+    import numpy as np
+    import torch
+
+    from gaussian_splatting_b200 import synth
+
+    spec = importlib.util.spec_from_file_location("bench_module", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    n = bench.DUMP_ROWS + 1000
+    g = synth.make_gaussians(n, "tiny", sh_degree=bench.SH_DEGREE, seed=0, requires_grad=True)
+    for p in (g.xyz, g.rgb, g.opacity, g.scale, g.quaternion, g.sh):
+        p.grad = torch.randn_like(p)
+    mask = torch.rand(n, generator=torch.Generator().manual_seed(0)) < 0.3
+    uv = torch.randn(int((~mask).sum()), 2)
+    image = torch.rand(1080, 1920, 3)
+    names = bench.dump_outputs(tmp_path / "a", image, mask, uv, g)
+    bench.dump_outputs(tmp_path / "b", image, mask, uv, g)
+    total = 0
+    for name in names:
+        a = np.load(tmp_path / "a" / f"{name}.npy")
+        assert a.dtype in (np.float32, np.float64), name
+        assert np.isfinite(a).all(), name
+        assert np.array_equal(a, np.load(tmp_path / "b" / f"{name}.npy")), name
+        total += (tmp_path / "a" / f"{name}.npy").stat().st_size
+    assert total <= 64 * 2**20, total
+    rows = np.load(tmp_path / "a" / "gaussian_rows.npy").astype(np.int64)
+    culled = np.load(tmp_path / "a" / "culling_mask.npy")
+    assert culled.tolist() == mask[rows].float().tolist() and culled.any()
+    uv_rows = np.load(tmp_path / "a" / "uv.npy")
+    assert (uv_rows[culled == 1] == 0).all()
+    uv_all = np.zeros((n, 2), np.float32)
+    uv_all[~mask.numpy()] = uv.numpy()
+    assert np.array_equal(uv_rows, uv_all[rows])

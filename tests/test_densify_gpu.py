@@ -2,12 +2,12 @@
 
   1. the native apply pass against a torch-indexing stand-in of the same plan, bit for bit;
   2. AdaptiveDensityControl (plan + native apply on FlatAdam's buffers) against the reference's UNMODIFIED trainer
-     code (oracle/_ref: splat_py/trainer.py `adaptive_density_control` with splat_py/optimizer_manager.py on
-     torch.optim.Adam) on a 100k-gaussian scene: identical surviving / cloned / split rows, bit-identical
-     parameters and Adam moments."""
-import sys
-import types
+     code (splat_py/trainer.py `adaptive_density_control` with splat_py/optimizer_manager.py on torch.optim.Adam,
+     tests/golden/ref_densify_trainer.npz) on a 100k-gaussian scene: identical surviving / cloned / split rows,
+     bit-identical parameters and Adam moments."""
+from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 
@@ -15,7 +15,7 @@ from gaussian_splatting_b200.densify import (AdaptiveDensityControl, Densificati
                                              plan_adaptive_density_control)
 from gaussian_splatting_b200.flat_adam import FIELDS, REFERENCE_LR_MULTIPLIERS, FlatAdam
 from gaussian_splatting_b200.structs import Gaussians
-from oracle import ref_loader
+from tests import scenes
 from tests.test_densify_plan import emulate_apply, make_case
 
 pytestmark = pytest.mark.gpu
@@ -72,31 +72,12 @@ def test_native_apply_matches_indexing_bitwise(n):
     opt.step(torch.zeros_like(opt.p))
 
 
-@pytest.mark.skipif(not (ref_loader.REF_DIR / "splat_py" / "trainer.py").exists(), reason="oracle/_ref not present")
 def test_adaptive_density_control_matches_the_reference_trainer():
-    ref_loader.load_reference_trainer()
-    RT = sys.modules["splat_py_trainer_ref.trainer"]
-    RC = sys.modules["splat_py_trainer_ref.config"]
-    RO = sys.modules["splat_py_trainer_ref.optimizer_manager"]
-    RS = sys.modules["splat_py_trainer_ref.structs"]
+    """Two passes on make_case(100_000, seed=21): after each, every parameter and both Adam moments hold the values
+    the reference trainer computed from the same case and seeds (value digests, tools/make_golden.py --sets densify)."""
+    gd = np.load(Path(__file__).resolve().parent / "golden" / "ref_densify_trainer.npz")
     n = 100_000
     P, M, V, uv_acc, xyz_acc, cnt = make_case(n, seed=21, device=dev(), n_rest=15)
-    config = RC.SplatConfig()
-
-    # --- the reference: nn.Parameters + torch.optim.Adam with populated state, its own trainer methods
-    gr = RS.Gaussians(*(torch.nn.Parameter(P[k].clone()) for k in ("xyz", "rgb", "opacity", "scale", "quaternion")),
-                      sh=torch.nn.Parameter(P["sh"].clone()))
-    trainer = object.__new__(RT.SplatTrainer)
-    trainer.gaussians, trainer.config = gr, config
-    trainer.optimizer_manager = RO.OptimizerManager(gr, config)
-    order = ("xyz", "quaternion", "scale", "opacity", "rgb", "sh")  # optimizer_manager.py:13-44 group order
-    for k, group in zip(order, trainer.optimizer_manager.optimizer.param_groups):
-        p = group["params"][0]
-        trainer.optimizer_manager.optimizer.state[p] = dict(step=torch.tensor(7.0), exp_avg=M[k].clone(),
-                                                            exp_avg_sq=V[k].clone())
-    trainer.uv_grad_accum, trainer.xyz_grad_accum, trainer.grad_accum_count = uv_acc.clone(), xyz_acc.clone(), cnt.clone()
-
-    # --- this library: flat buffers
     g, opt = flat_setup(P, M, V)
     stats = DensificationStats(n, dev())
     stats.uv_grad_accum, stats.xyz_grad_accum, stats.grad_accum_count = uv_acc.clone(), xyz_acc.clone(), cnt.clone()
@@ -104,27 +85,22 @@ def test_adaptive_density_control_matches_the_reference_trainer():
 
     for it in (800, 900):  # two consecutive passes: the second one runs on the first one's output
         torch.manual_seed(100 + it)
-        trainer.adaptive_density_control(it)
-        torch.manual_seed(100 + it)
         info = adc.adaptive_density_control(it)
         assert info["deleted"] > 0 or it != 800
-        assert g.xyz.shape[0] == gr.xyz.shape[0], info
-        state = trainer.optimizer_manager.optimizer.state
-        groups = trainer.optimizer_manager.optimizer.param_groups
+        assert g.xyz.shape[0] == int(gd[f"it{it}_n"]), info
         m_sec, v_sec = sections(opt, g, opt.m), sections(opt, g, opt.v)
-        for k, group in zip(order, groups):
-            p = group["params"][0]
-            assert torch.equal(getattr(g, k).detach(), getattr(gr, k).detach()), (it, k)
-            assert torch.equal(m_sec[k], state[p]["exp_avg"]) and torch.equal(v_sec[k], state[p]["exp_avg_sq"]), (it, k)
-        assert stats.grad_accum_count.shape[0] == trainer.grad_accum_count.shape[0]
-        # new statistics for the next pass (both sides the same)
+        for k in ("xyz", "quaternion", "scale", "opacity", "rgb", "sh"):
+            assert scenes.value_digest(getattr(g, k)) == str(gd[f"it{it}_{k}"]), (it, k)
+            assert scenes.value_digest(m_sec[k]) == str(gd[f"it{it}_{k}_exp_avg"]), (it, k)
+            assert scenes.value_digest(v_sec[k]) == str(gd[f"it{it}_{k}_exp_avg_sq"]), (it, k)
+        assert stats.grad_accum_count.shape[0] == int(gd[f"it{it}_count_rows"])
+        # new statistics for the next pass (the reference was given the same)
         n_now = g.xyz.shape[0]
         gen = torch.Generator(device=dev()).manual_seed(it)
         uv2 = torch.rand(n_now, 2, device=dev(), generator=gen) * 1e-3
         xyz2 = torch.rand(n_now, 3, device=dev(), generator=gen) * 1e-3
         cnt2 = torch.randint(0, 4, (n_now,), device=dev(), generator=gen, dtype=torch.int32)
         uv2[cnt2 == 0] = 0.0
-        trainer.uv_grad_accum, trainer.xyz_grad_accum, trainer.grad_accum_count = uv2.clone(), xyz2.clone(), cnt2.clone()
         stats.uv_grad_accum, stats.xyz_grad_accum, stats.grad_accum_count = uv2.clone(), xyz2.clone(), cnt2.clone()
 
 

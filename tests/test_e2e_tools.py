@@ -1,12 +1,14 @@
-"""tools/e2e (reference trainer on a synthetic COLMAP scene): the scene writer's binary files are read back by the
-reference's own COLMAP reader (installed copy under oracle/_ref), and the SSIM stand-in behaves like an SSIM."""
+"""tools/e2e (reference trainer on a synthetic COLMAP scene): the scene writer's binary files are the ones the
+reference's own COLMAP reader read back correctly (tests/golden/ref_colmap_reader.npz), and the SSIM stand-in
+behaves like an SSIM."""
 import importlib.util
 import sys
 from pathlib import Path
 
 import numpy as np
-import pytest
 import torch
+
+from tests import scenes
 
 ROOT = Path(__file__).resolve().parents[1]
 E2E = ROOT / "tools" / "e2e"
@@ -20,29 +22,31 @@ def _load(path, name):
 
 
 def test_colmap_writers_round_trip_through_the_reference_reader(tmp_path):
-    reader_py = ROOT / "oracle" / "_ref" / "splat_py" / "read_colmap.py"
-    if not reader_py.exists():
-        pytest.skip("oracle/_ref (installed reference) not present")
-    rd = _load(reader_py, "ref_read_colmap")
+    """The writers still write the files the reference's reader was given (bytes equal, float64 fields to 1e-12),
+    and what the reader returned from them is the scene that was written."""
+    gd = np.load(ROOT / "tests" / "golden" / "ref_colmap_reader.npz")
     mk = _load(E2E / "make_colmap_scene.py", "make_colmap_scene")
-    poses = [mk.look_at(np.array([4 * np.cos(a), 4 * np.sin(a), 1.2 + 0.8 * np.sin(3 * a)])) for a in np.linspace(0, 6.2, 17)]
-    names = [f"view_{i:03d}.png" for i in range(len(poses))]
+    poses, names, xyz, rgb = scenes.colmap_scene(mk)
     mk.write_cameras(tmp_path / "cameras.bin", 640, 416, 560.0, 561.0, 320.0, 208.0)
     mk.write_images(tmp_path / "images.bin", poses, names)
-    xyz = np.random.default_rng(0).standard_normal((50, 3))
-    rgb = np.random.default_rng(1).integers(0, 256, (50, 3)).astype(np.uint8)
     mk.write_points(tmp_path / "points3D.bin", xyz, rgb)
-    cams = rd.read_cameras_binary(str(tmp_path / "cameras.bin"))
-    assert cams[1].model == "PINHOLE" and (cams[1].width, cams[1].height) == (640, 416)
-    assert np.allclose(cams[1].params, [560.0, 561.0, 320.0, 208.0])
-    imgs = rd.read_images_binary(str(tmp_path / "images.bin"))
-    assert len(imgs) == len(poses)
-    for i, T in enumerate(poses, start=1):
-        assert imgs[i].name == names[i - 1] and imgs[i].camera_id == 1
-        assert np.abs(rd.qvec2rotmat(imgs[i].qvec) - T[:3, :3]).max() < 1e-12
-        assert np.abs(imgs[i].tvec - T[:3, 3]).max() < 1e-12
-    pts = rd.read_points3D_binary(str(tmp_path / "points3D.bin"))
-    assert len(pts) == 50 and np.allclose(pts[7].xyz, xyz[6]) and (pts[7].rgb == rgb[6]).all()
+    for f in ("cameras", "images", "points3D"):
+        got, ref = np.frombuffer((tmp_path / f"{f}.bin").read_bytes(), np.uint8), gd[f + "_bytes"]
+        assert got.shape == ref.shape, f
+        fields = (gd[f + "_f64_at"][:, None] + np.arange(8)).ravel()
+        rest = np.ones(ref.size, bool)
+        rest[fields] = False
+        assert (got[rest] == ref[rest]).all(), f
+        assert np.abs(got[fields].view("<f8") - ref[fields].view("<f8")).max() <= 1e-12, f
+    assert gd["cam_ids"].tolist() == [1] and gd["cam_model"].tolist() == ["PINHOLE"]
+    assert gd["cam_size"][0].tolist() == [640, 416] and np.allclose(gd["cam_params"][0], [560.0, 561.0, 320.0, 208.0])
+    assert gd["img_ids"].tolist() == list(range(1, len(poses) + 1))
+    for i, T in enumerate(poses):
+        assert gd["img_names"][i] == names[i] and gd["img_camera_ids"][i] == 1
+        assert np.abs(gd["img_rotmat"][i] - T[:3, :3]).max() < 1e-12
+        assert np.abs(gd["img_tvec"][i] - T[:3, 3]).max() < 1e-12
+    assert gd["pt_ids"].tolist() == list(range(1, 51))
+    assert np.allclose(gd["pt_xyz"][6], xyz[6]) and (gd["pt_rgb"][6] == rgb[6]).all()
 
 
 def test_ssim_shim_is_an_ssim():

@@ -5,7 +5,9 @@ Three independent checkers, strongest first:
      Forward quantities must match BIT FOR BIT (uv, conic, tile lists, image, per-pixel state);
      gradients within max(1e-4, 10 x the reference's own run-to-run noise) of max|ref| (fp32 atomics
      make the reference itself nondeterministic, SURVEY.md Q18).
-  2. oracle/_ref live, when the compiled reference travelled with the tree (same assertions, bigger scene).
+  2. tests/golden/ref_*.npz — what the compiled reference computed on bigger scenes (100k and 3M gaussians):
+     forward quantities as bit digests, gradients as seeded row samples with max|ref| (tests/scenes.py);
+     the drop-in test runs the reference's own python on this library when oracle/_ref is built.
   3. the CPU oracle (oracle/cpu_oracle.py), tolerance 1e-4 rel fp32 (north_star), which differs from the
      GPU only in the transcendental functions.
 plus size-independent properties at BASELINE.json's full size (1080p, 3M gaussians).
@@ -56,6 +58,11 @@ def assert_bits_equal(a, b, what):
     assert ba.shape == bb.shape, (what, ba.shape, bb.shape)
     bad = int((ba != bb).sum())
     assert bad == 0, f"{what}: {bad}/{ba.size} values differ bitwise from the reference"
+
+
+def assert_digest(a, gd, key, what):
+    """Bit-for-bit comparison with a reference array the fixture keeps as a digest (key + "_sha")."""
+    assert scenes.bits_digest(a) == str(gd[key + "_sha"]), f"{what}: bits differ from the reference's"
 
 
 def gaussians_from(sc, requires_grad=True):
@@ -229,165 +236,92 @@ def test_golden_fp64_operator_surface(n_sh):
 
 
 # ------------------------------------------------------------------------------------------------
-# 2. the compiled reference, live (only when oracle/_ref travelled with the tree)
+# 2. the compiled reference on bigger scenes (tests/golden/ref_*.npz, tools/make_golden.py --sets comparisons)
 # ------------------------------------------------------------------------------------------------
 needs_ref = pytest.mark.skipif(not ref_loader.reference_available(), reason="oracle/_ref not present")
+GRADS = ("g_xyz", "g_rgb", "g_opacity", "g_scale", "g_quaternion", "g_sh", "g_uv")
 
 
-@needs_ref
 @pytest.mark.parametrize("pose", ["yaw", "general"])
 def test_live_reference_100k_720p(pose):
-    ref_loader.load_reference()
-    ref_ras = sys.modules["splat_py_ref.rasterize"]
-    ref_structs = sys.modules["splat_py_ref.structs"]
-    sc = scenes.np_scene(100_000, "720p", sh_degree=3, seed=0, view=0, n_views=3)
-    if pose == "general":
-        c, s = np.cos(0.3), np.sin(0.3)
-        R = np.array([[c, -s, 0], [s, c, 0], [0, 0, 1]], np.float64) @ np.array([[1, 0, 0], [0, 0.995, -0.0998], [0, 0.0998, 0.995]])
-        T = np.eye(4)
-        T[:3, :3], T[:3, 3] = R, [0.13, -0.21, 0.37]
-        sc["T"] = T.astype(np.float32)
-    G = synth.make_upstream_grad("720p").numpy()
-    mine = run_b200(sc, G=G)
-    g = gaussians_from(sc)
-    gr = ref_structs.Gaussians(g.xyz, g.rgb, g.opacity, g.scale, g.quaternion, g.sh)
-    image, mask, uv = ref_ras.rasterize(gr, to_t(sc["T"]), ref_structs.Camera(sc["W"], sc["H"], to_t(sc["K"])),
-                                        0.3, 500.0, 100, 3.0, True, torch.full((3,), 0.5, device=dev()))
-    uv.retain_grad()
-    image.backward(to_t(G))
-    assert_bits_equal(mine["culling_mask"], mask, "culling_mask")
-    assert_bits_equal(mine["uv"], uv, "uv")
-    assert_bits_equal(mine["image"], image, "image")
-    for k, v in dict(g_xyz=g.xyz.grad, g_rgb=g.rgb.grad, g_opacity=g.opacity.grad, g_scale=g.scale.grad,
-                     g_quaternion=g.quaternion.grad, g_sh=g.sh.grad, g_uv=uv.grad).items():
-        assert rel(mine[k], v) < REL_TOL, (k, rel(mine[k], v))
+    """100k gaussians, SH 3, 720p, the synthetic yaw pose and a general one: forward bit for bit with the compiled
+    reference, gradients within 1e-4 of max|ref|."""
+    gd = load_golden("ref_live_100k_720p.npz")
+    mine = run_b200(scenes.live_720p_scene(pose), G=synth.make_upstream_grad("720p").numpy())
+    for k in ("culling_mask", "uv", "image"):
+        assert_digest(mine[k], gd, f"{pose}_{k}", k)
+    for k in GRADS:
+        assert scenes.rel_rows(mine[k], gd, f"{pose}_{k}") < REL_TOL, (k, scenes.rel_rows(mine[k], gd, f"{pose}_{k}"))
 
 
-@needs_ref
 def test_live_reference_exact_arithmetic_paths():
     """Scene built to hit the forward kernel's rare exact paths (DESIGN.md 3.1): splats whose centre falls
     EXACTLY on a pixel centre (numerator 0, outside the hoisted-reciprocal division's proven range) and splats
     whose 2-D covariance determinant exceeds 1e18 (record marked unsafe) — the flagged pixels are recomputed by
     render_pixel_exact_warp.  Everything must still match the compiled reference bit for bit."""
-    ref_loader.load_reference()
-    ref_ras = sys.modules["splat_py_ref.rasterize"]
-    ref_structs = sys.modules["splat_py_ref.structs"]
-    rng = np.random.default_rng(7)
-    sc = scenes.np_scene(3000, "tiny", sh_degree=0, seed=3, sigma_px=(2.0, 0.5, 0.5, 8.0))
-    sc["K"] = np.array([[64, 0, 32], [0, 64, 32], [0, 0, 1]], np.float32)  # powers of two: u = 64*x/z + 32 is exact
-    sc["T"] = np.eye(4, dtype=np.float32)
-    n_exact, n_huge = 300, 12
-    z = np.full(n_exact, 2.0, np.float32)
-    px, py = rng.integers(0, 64, n_exact), rng.integers(0, 64, n_exact)
-    sc["xyz"][:n_exact] = np.stack([(px - 32) / 64.0 * z, (py - 32) / 64.0 * z, z], 1).astype(np.float32)
-    sc["xyz"][n_exact:n_exact + n_huge, 2] = 2.0
-    sc["scale"][n_exact:n_exact + n_huge] = 7.5       # exp(7.5) = 1808 world units -> det(Sigma_2D) ~ 1e19
-    sc["opacity"][n_exact:n_exact + n_huge] = -3.0
-    G = synth.make_upstream_grad("tiny").numpy()
-    mine = run_b200(sc, G=G)
-    g = gaussians_from(sc)
-    gr = ref_structs.Gaussians(g.xyz, g.rgb, g.opacity, g.scale, g.quaternion, g.sh)
-    image, mask, uv = ref_ras.rasterize(gr, to_t(sc["T"]), ref_structs.Camera(64, 64, to_t(sc["K"])), 0.3, 500.0, 100, 3.0,
-                                        True, torch.full((3,), 0.5, device=dev()))
-    uv.retain_grad()
-    image.backward(to_t(G))
-    uvn = uv.detach().cpu().numpy()
-    assert int(((uvn == np.round(uvn)).all(1)).sum()) >= n_exact // 2   # the exact-centre splats survived culling
-    assert_bits_equal(mine["culling_mask"], mask, "culling_mask")
-    assert_bits_equal(mine["uv"], uv, "uv")
-    assert_bits_equal(mine["image"], image, "image")
-    for k, v in dict(g_xyz=g.xyz.grad, g_rgb=g.rgb.grad, g_opacity=g.opacity.grad, g_scale=g.scale.grad,
-                     g_quaternion=g.quaternion.grad, g_uv=uv.grad).items():
-        assert rel(mine[k], v) < REL_TOL, (k, rel(mine[k], v))
+    gd = load_golden("ref_exact_paths_tiny.npz")
+    mine = run_b200(scenes.exact_paths_scene(), G=synth.make_upstream_grad("tiny").numpy())
+    uvn = gd["uv"]
+    assert int(((uvn == np.round(uvn)).all(1)).sum()) >= scenes.EXACT_PATHS_N_EXACT // 2  # exact centres survived culling
+    assert_bits_equal(mine["culling_mask"], gd["culling_mask"], "culling_mask")
+    assert_bits_equal(mine["uv"], gd["uv"], "uv")
+    assert_bits_equal(mine["image"], gd["image"], "image")
+    for k in ("g_xyz", "g_rgb", "g_opacity", "g_scale", "g_quaternion", "g_uv"):
+        assert rel(mine[k], gd[k]) < REL_TOL, (k, rel(mine[k], gd[k]))
 
 
-@needs_ref
 @pytest.mark.parametrize("H", [1080, 1088])
 def test_live_reference_3M_headline(H):
-    """BASELINE.json configs[2] under the driver's tests: 3M gaussians, SH 3, 1920 x H against the compiled
-    reference on the same device.  H = 1080 is the headline; H = 1088 (a multiple of 16) is the strict run,
-    because at H % 16 != 0 the reference's forward has a barrier inside `if (valid_pixel)` (src/render.cu:101,164,
-    SURVEY.md Q15) and its bottom tile row is racy for tiles with more than one 960-splat chunk.  Forward
-    quantities bit for bit (bottom tile row of H = 1080: only where the reference agrees with itself); gradients
-    within max(1e-4, 10 x the reference's own run-to-run noise) of max|ref|."""
-    ref_loader.load_reference()
-    ref_ras = sys.modules["splat_py_ref.rasterize"]
-    ref_structs = sys.modules["splat_py_ref.structs"]
+    """BASELINE.json configs[2]: 3M gaussians, SH 3, 1920 x H against the compiled reference.  H = 1080 is the
+    headline; H = 1088 (a multiple of 16) is the strict run, because at H % 16 != 0 the reference's forward has a
+    barrier inside `if (valid_pixel)` (src/render.cu:101,164, SURVEY.md Q15) and its bottom tile row is racy for
+    tiles with more than one 960-splat chunk.  Forward quantities bit for bit (bottom tile row of H = 1080: only
+    where the reference agreed with itself over two runs); gradients within max(1e-4, 10 x the reference's own
+    run-to-run noise) of max|ref|."""
+    gd = load_golden("ref_headline_3M.npz")
+    p = f"h{H}_"
     d = dev()
     names = ("xyz", "quaternion", "scale", "opacity", "rgb", "sh")
     g = synth.make_gaussians(3_000_000, "1080p", sh_degree=3, seed=0, device=d, requires_grad=True)
-    cam0 = synth.make_camera("1080p", device=d)
-    cam = Camera(1920, H, cam0.K)
+    cam = Camera(1920, H, synth.make_camera("1080p", device=d).K)
     T = synth.make_pose(2, 8, device=d)
     bg = torch.full((3,), 0.5, device=d)
-    gen = torch.Generator().manual_seed(1)
-    G = (torch.randn(H, 1920, 3, generator=gen, dtype=torch.float64) / (3.0 * H * 1920)).float().to(d)
-
-    def grads_and_clear():
-        out = {k: getattr(g, k).grad.clone() for k in names}
-        for k in names:
-            getattr(g, k).grad = None
-        return out
+    G = scenes.headline_upstream_grad(H).to(d)
 
     image, mask, uv, st = rasterize(g, T, cam, 0.3, 500.0, 100, 3.0, True, bg, return_state=True)
     uv.retain_grad()
     image.backward(G)
-    mine, mine_uv = grads_and_clear(), uv.grad.clone()
-    image, uv_mine = image.detach(), uv.detach()
     n_mine, w_mine, ranges = st.n_per_pixel, st.w_per_pixel, st.ranges
     del st
 
-    gr = ref_structs.Gaussians(g.xyz, g.rgb, g.opacity, g.scale, g.quaternion, g.sh)
-    camr = ref_structs.Camera(1920, H, cam0.K)
-    runs = []
-    for _ in range(2):  # twice: the reference's own nondeterminism (fp32 atomics, Q15 / Q18) is the noise floor
-        im, mk, uvr = ref_ras.rasterize(gr, T, camr, 0.3, 500.0, 100, 3.0, True, bg)
-        uvr.retain_grad()
-        im.backward(G)
-        runs.append((im.detach(), mk, uvr.detach(), grads_and_clear(), uvr.grad.clone()))
-    (im_a, mask_r, uv_r, gr_a, guv_a), (im_b, _, _, gr_b, guv_b) = runs
-
-    assert_bits_equal(mask, mask_r, "culling_mask")
-    assert_bits_equal(uv_mine, uv_r, "uv")
+    assert_digest(mask, gd, p + "culling_mask", "culling_mask")
+    assert_digest(uv, gd, p + "uv", "uv")
     body = (H // 16) * 16
-    assert_bits_equal(image[:body], im_a[:body], "image (full tile rows)")
-    if body < H:  # ragged bottom tile row: judge only the pixels where the reference reproduces itself
-        stable = (im_a[body:] == im_b[body:]).all(dim=2)
+    assert_digest(image[:body], gd, p + "image_body", "image (full tile rows)")
+    if body < H:  # ragged bottom tile row: judge only the pixels where the reference reproduced itself
+        stable = torch.from_numpy(gd[p + "bottom_stable"]).to(d)
         assert float(stable.float().mean()) > 0.5
-        assert_bits_equal(image[body:][stable], im_a[body:][stable], "image (bottom tile row, race-free pixels)")
+        assert_digest(image[body:][stable], gd, p + "bottom_stable", "image (bottom tile row, race-free pixels)")
     cnt = (ranges[1:] - ranges[:-1]).view((H + 15) // 16, 120)
     assert bool((n_mine <= cnt.repeat_interleave(16, 0).repeat_interleave(16, 1)[:H, :1920]).all())
     assert bool(torch.isfinite(w_mine).all())
-    for k in names:
-        noise = rel(gr_b[k], gr_a[k])
+    for k, got in [(f"g_{k}", getattr(g, k).grad) for k in names] + [("g_uv", uv.grad)]:
+        noise = float(gd[p + "noise_" + k])
         tol = max(REL_TOL, 10.0 * noise)
-        assert rel(mine[k], gr_a[k]) < tol, (k, rel(mine[k], gr_a[k]), noise)
-    assert rel(mine_uv, guv_a) < max(REL_TOL, 10.0 * rel(guv_b, guv_a))
+        assert scenes.rel_rows(got, gd, p + k) < tol, (k, scenes.rel_rows(got, gd, p + k), noise)
 
 
-@needs_ref
 def test_live_reference_per_pixel_sh_backward_fp32():
     """use_sh_precompute=False (per-pixel view directions, N_SH = 16) in fp32, forward AND backward against the
     compiled reference (src/render.cu:284-333, src/render_backward.cu:402-568): the golden fixtures pin the fp32
     image and the fp64 gradients of this mode, this pins the fp32 gradients."""
-    ref_loader.load_reference()
-    ref_ras = sys.modules["splat_py_ref.rasterize"]
-    ref_structs = sys.modules["splat_py_ref.structs"]
-    sc = scenes.np_scene(20_000, "small", sh_degree=3, seed=5, view=1, n_views=3, sigma_px=(2.5, 0.5, 0.5, 10.0))
-    G = synth.make_upstream_grad("small").numpy()
-    mine = run_b200(sc, G=G, sh_precompute=False)
-    g = gaussians_from(sc)
-    gr = ref_structs.Gaussians(g.xyz, g.rgb, g.opacity, g.scale, g.quaternion, g.sh)
-    image, mask, uv = ref_ras.rasterize(gr, to_t(sc["T"]), ref_structs.Camera(sc["W"], sc["H"], to_t(sc["K"])),
-                                        0.3, 500.0, 100, 3.0, False, torch.full((3,), 0.5, device=dev()))
-    uv.retain_grad()
-    image.backward(to_t(G))
-    assert_bits_equal(mine["culling_mask"], mask, "culling_mask")
-    assert_bits_equal(mine["uv"], uv, "uv")
-    assert rel(mine["image"], image) < 1e-5
-    for k, v in dict(g_xyz=g.xyz.grad, g_rgb=g.rgb.grad, g_opacity=g.opacity.grad, g_scale=g.scale.grad,
-                     g_quaternion=g.quaternion.grad, g_sh=g.sh.grad, g_uv=uv.grad).items():
-        assert rel(mine[k], v) < REL_TOL, (k, rel(mine[k], v))
+    gd = load_golden("ref_per_pixel_sh_small.npz")
+    mine = run_b200(scenes.per_pixel_sh_scene(), G=synth.make_upstream_grad("small").numpy(), sh_precompute=False)
+    assert_digest(mine["culling_mask"], gd, "culling_mask", "culling_mask")
+    assert_digest(mine["uv"], gd, "uv", "uv")
+    assert rel(mine["image"], gd["image"]) < 1e-5
+    for k in GRADS:
+        assert scenes.rel_rows(mine[k], gd, k) < REL_TOL, (k, scenes.rel_rows(mine[k], gd, k))
 
 
 def test_contribution_masks_do_not_change_the_gradients():

@@ -1,10 +1,17 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (oracle/_ref: its CUDA extension +
-its splat_py package) on a B200.  Run on the GPU box:
+its splat_py package, built by oracle/build_ref.py) on a B200:
 
-    gpurun -- python tools/make_golden.py --out gpurun_out/golden      # then copy into tests/golden/
+    python tools/make_golden.py --out <dir> [--sets fixtures comparisons densify colmap]   # then copy into tests/golden/
 
 Scenes are regenerated from seeds by the tests (gaussian_splatting_b200.synth / tests/scenes.py); the
 fixtures hold only the reference's OUTPUTS.  Nothing here touches the product code.
+
+  fixtures     fixture6 / synth_* : per-operator outputs, images and gradients of small scenes
+  comparisons  ref_*.npz : what the tests comparing with the reference at 100k / 3M gaussians check, in the
+               compact forms of tests/scenes.py (bit digests, seeded row samples of the gradients)
+  densify      ref_densify_trainer.npz : the reference trainer's densification of a 100k-gaussian case
+  colmap       ref_colmap_reader.npz : files of tools/e2e/make_colmap_scene.py and what the reference's
+               COLMAP reader read from them (CPU only)
 """
 from __future__ import annotations
 
@@ -100,16 +107,7 @@ def render_state(ref_ext, st, sc, dev, bg):
     return dict(num_splats_per_pixel=n(npp).astype(np.int32), final_weight_per_pixel=n(wl), image_from_stages=n(img))
 
 
-def main():
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default="gpurun_out/golden")
-    args = ap.parse_args()
-    out = Path(args.out)
-    out.mkdir(parents=True, exist_ok=True)
-    dev = torch.device("cuda")
-    ref_ext, _ = ref_loader.load_reference()
-    meta = dict(gpu=torch.cuda.get_device_name(0), torch=torch.__version__)
-
+def fixtures(out, dev, ref_ext, meta):
     # A. the reference's own 6-gaussian unit-test scene (test/gaussian_test_data.py)
     fx = scenes.reference_fixture()
     stA = stages(ref_ext, fx, dev, near=0.3, far=100.0, pad=10, mh=3.0)
@@ -185,6 +183,197 @@ def main():
         d64.update({f"nsh{n_sh}_image": n(image), f"nsh{n_sh}_sorted_idx": n(sidx), f"nsh{n_sh}_ranges": n(rng),
                     **{f"nsh{n_sh}_g_{k}": n(v.grad) for k, v in P.items() if v.grad is not None}})
     np.savez_compressed(out / "synth_tiny_fp64.npz", **d64)
+
+
+GRADS = ("g_xyz", "g_rgb", "g_opacity", "g_scale", "g_quaternion", "g_sh")
+
+
+def keep_comparison(d, prefix, r, seed):
+    """One reference run `r` (run_rasterize with gradients): forward outputs as bit digests, gradients as seeded
+    samples of the visible gaussians' rows (g_uv: of all its rows)."""
+    for k in ("culling_mask", "uv", "image"):
+        d[f"{prefix}{k}_sha"] = np.array(scenes.bits_digest(r[k]))
+    visible = np.flatnonzero(~r["culling_mask"])
+    for k in GRADS:
+        if k in r:
+            scenes.keep_rows(d, prefix + k, r[k], visible, seed)
+    scenes.keep_rows(d, prefix + "g_uv", r["g_uv"], np.arange(len(r["g_uv"])), seed)
+
+
+def comparisons(out, dev, meta):
+    d = {}
+    G = synth.make_upstream_grad("720p").numpy()
+    for pose in ("yaw", "general"):
+        r = run_rasterize(None, scenes.live_720p_scene(pose), dev, True, 0.5, G)
+        keep_comparison(d, pose + "_", r, seed=0)
+    np.savez_compressed(out / "ref_live_100k_720p.npz", **d)
+
+    # small enough to keep whole
+    r = run_rasterize(None, scenes.exact_paths_scene(), dev, True, 0.5, synth.make_upstream_grad("tiny").numpy())
+    np.savez_compressed(out / "ref_exact_paths_tiny.npz", **r)
+
+    r = run_rasterize(None, scenes.per_pixel_sh_scene(), dev, False, 0.5, synth.make_upstream_grad("small").numpy())
+    d = dict(image=r["image"])
+    for k in ("culling_mask", "uv"):
+        d[k + "_sha"] = np.array(scenes.bits_digest(r[k]))
+    visible = np.flatnonzero(~r["culling_mask"])
+    for k in GRADS:
+        scenes.keep_rows(d, k, r[k], visible, seed=0)
+    scenes.keep_rows(d, "g_uv", r["g_uv"], np.arange(len(r["g_uv"])), seed=0)
+    np.savez_compressed(out / "ref_per_pixel_sh_small.npz", **d)
+
+    # 3M gaussians, SH 3, 1920 x H, pose 2 of 8; the reference twice: its run-to-run noise sets the gradient tolerance
+    ras, structs = sys.modules["splat_py_ref.rasterize"], sys.modules["splat_py_ref.structs"]
+    names = ("xyz", "quaternion", "scale", "opacity", "rgb", "sh")
+    d = {}
+    for H in (1080, 1088):
+        g = synth.make_gaussians(3_000_000, "1080p", sh_degree=3, seed=0, device=dev, requires_grad=True)
+        gr = structs.Gaussians(g.xyz, g.rgb, g.opacity, g.scale, g.quaternion, g.sh)
+        camr = structs.Camera(1920, H, synth.make_camera("1080p", device=dev).K)
+        T, bg, G = synth.make_pose(2, 8, device=dev), torch.full((3,), 0.5, device=dev), scenes.headline_upstream_grad(H).to(dev)
+        runs = []
+        for _ in range(2):
+            im, mk, uvr = ras.rasterize(gr, T, camr, 0.3, 500.0, 100, 3.0, True, bg)
+            uvr.retain_grad()
+            im.backward(G)
+            grads = {k: getattr(g, k).grad.clone() for k in names}
+            for k in names:
+                getattr(g, k).grad = None
+            runs.append((im.detach(), mk, uvr.detach(), grads, uvr.grad.clone()))
+        (im_a, mask, uv, gr_a, guv_a), (im_b, _, _, gr_b, guv_b) = runs
+        p = f"h{H}_"
+        d[p + "culling_mask_sha"], d[p + "uv_sha"] = np.array(scenes.bits_digest(mask)), np.array(scenes.bits_digest(uv))
+        body = (H // 16) * 16
+        d[p + "image_body_sha"] = np.array(scenes.bits_digest(im_a[:body]))
+        if body < H:  # ragged bottom tile row: only the pixels where the reference reproduces itself
+            stable = (im_a[body:] == im_b[body:]).all(dim=2)
+            d[p + "bottom_stable"] = n(stable)
+            d[p + "bottom_stable_sha"] = np.array(scenes.bits_digest(im_a[body:][stable]))
+        visible = np.flatnonzero(~n(mask))
+        rel = lambda a, b: float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))  # noqa: E731
+        for k in names:
+            d[p + "noise_g_" + k] = np.float64(rel(gr_b[k], gr_a[k]))
+            scenes.keep_rows(d, p + "g_" + k, n(gr_a[k]), visible, seed=H)
+        d[p + "noise_g_uv"] = np.float64(rel(guv_b, guv_a))
+        scenes.keep_rows(d, p + "g_uv", n(guv_a), np.arange(guv_a.shape[0]), seed=H)
+        meta[f"headline_{H}"] = {k: float(v) for k, v in d.items() if k.startswith(p + "noise")}
+        del g, gr, runs, im_a, im_b, gr_a, gr_b
+        torch.cuda.empty_cache()
+    np.savez_compressed(out / "ref_headline_3M.npz", **d)
+
+
+def densify(out, dev, meta):
+    """The reference trainer's adaptive_density_control (trainer.py + optimizer_manager.py on torch.optim.Adam with
+    populated state) on tests/test_densify_plan.make_case(100_000, seed=21), two passes; per pass the value digests
+    of every parameter and both Adam moments."""
+    from tests.test_densify_plan import make_case
+
+    ref_loader.load_reference_trainer()
+    RT, RC = sys.modules["splat_py_trainer_ref.trainer"], sys.modules["splat_py_trainer_ref.config"]
+    RO, RS = sys.modules["splat_py_trainer_ref.optimizer_manager"], sys.modules["splat_py_trainer_ref.structs"]
+    n_g = 100_000
+    P, M, V, uv_acc, xyz_acc, cnt = make_case(n_g, seed=21, device=dev, n_rest=15)
+    config = RC.SplatConfig()
+    gr = RS.Gaussians(*(torch.nn.Parameter(P[k].clone()) for k in ("xyz", "rgb", "opacity", "scale", "quaternion")),
+                      sh=torch.nn.Parameter(P["sh"].clone()))
+    trainer = object.__new__(RT.SplatTrainer)
+    trainer.gaussians, trainer.config = gr, config
+    trainer.optimizer_manager = RO.OptimizerManager(gr, config)
+    order = ("xyz", "quaternion", "scale", "opacity", "rgb", "sh")  # optimizer_manager.py:13-44 group order
+    for k, group in zip(order, trainer.optimizer_manager.optimizer.param_groups):
+        trainer.optimizer_manager.optimizer.state[group["params"][0]] = dict(step=torch.tensor(7.0), exp_avg=M[k].clone(),
+                                                                             exp_avg_sq=V[k].clone())
+    trainer.uv_grad_accum, trainer.xyz_grad_accum, trainer.grad_accum_count = uv_acc, xyz_acc, cnt
+    d = {}
+    for it in (800, 900):
+        torch.manual_seed(100 + it)
+        trainer.adaptive_density_control(it)
+        state = trainer.optimizer_manager.optimizer.state
+        for k, group in zip(order, trainer.optimizer_manager.optimizer.param_groups):
+            p = group["params"][0]
+            d[f"it{it}_{k}"] = np.array(scenes.value_digest(getattr(gr, k)))
+            d[f"it{it}_{k}_exp_avg"] = np.array(scenes.value_digest(state[p]["exp_avg"]))
+            d[f"it{it}_{k}_exp_avg_sq"] = np.array(scenes.value_digest(state[p]["exp_avg_sq"]))
+        d[f"it{it}_n"] = np.int64(gr.xyz.shape[0])
+        d[f"it{it}_count_rows"] = np.int64(trainer.grad_accum_count.shape[0])
+        n_now = gr.xyz.shape[0]
+        gen = torch.Generator(device=dev).manual_seed(it)
+        uv2 = torch.rand(n_now, 2, device=dev, generator=gen) * 1e-3
+        xyz2 = torch.rand(n_now, 3, device=dev, generator=gen) * 1e-3
+        cnt2 = torch.randint(0, 4, (n_now,), device=dev, generator=gen, dtype=torch.int32)
+        uv2[cnt2 == 0] = 0.0
+        trainer.uv_grad_accum, trainer.xyz_grad_accum, trainer.grad_accum_count = uv2, xyz2, cnt2
+    meta["densify"] = {k: int(v) for k, v in d.items() if k.endswith("_n")}
+    np.savez_compressed(out / "ref_densify_trainer.npz", **d)
+
+
+def colmap(out, meta):
+    """tools/e2e/make_colmap_scene.py writes a scene; the reference's read_colmap.py reads it back.  Kept: the
+    files' bytes, the byte offsets of their float64 fields and what the reader returned."""
+    import importlib.util
+    import tempfile
+
+    def load(path, name):
+        spec = importlib.util.spec_from_file_location(name, str(path))
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)
+        return mod
+
+    rd = load(ref_loader.REF_DIR / "splat_py" / "read_colmap.py", "ref_read_colmap")
+    mk = load(ROOT / "tools" / "e2e" / "make_colmap_scene.py", "make_colmap_scene")
+    poses, names, xyz, rgb = scenes.colmap_scene(mk)
+    d = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        tmp = Path(tmp)
+        mk.write_cameras(tmp / "cameras.bin", 640, 416, 560.0, 561.0, 320.0, 208.0)
+        mk.write_images(tmp / "images.bin", poses, names)
+        mk.write_points(tmp / "points3D.bin", xyz, rgb)
+        for f in ("cameras", "images", "points3D"):
+            d[f + "_bytes"] = np.frombuffer((tmp / f"{f}.bin").read_bytes(), np.uint8)
+        cams = rd.read_cameras_binary(str(tmp / "cameras.bin"))
+        imgs = rd.read_images_binary(str(tmp / "images.bin"))
+        pts = rd.read_points3D_binary(str(tmp / "points3D.bin"))
+    # float64 fields: 8-byte header, then per record (make_colmap_scene.py write_*)
+    d["cameras_f64_at"] = np.array([32, 40, 48, 56])
+    at, o = [], 8
+    for name in names:
+        at += [o + 4 + 8 * j for j in range(7)]
+        o += 64 + len(name) + 1 + 8
+    d["images_f64_at"] = np.array(at)
+    d["points3D_f64_at"] = np.array([8 + 51 * i + j for i in range(len(xyz)) for j in (8, 16, 24, 35)])
+    d.update(cam_ids=np.array(sorted(cams)), cam_model=np.array([cams[i].model for i in sorted(cams)]),
+             cam_size=np.array([[cams[i].width, cams[i].height] for i in sorted(cams)]),
+             cam_params=np.array([cams[i].params for i in sorted(cams)]),
+             img_ids=np.array(sorted(imgs)), img_names=np.array([imgs[i].name for i in sorted(imgs)]),
+             img_camera_ids=np.array([imgs[i].camera_id for i in sorted(imgs)]),
+             img_rotmat=np.array([rd.qvec2rotmat(imgs[i].qvec) for i in sorted(imgs)]),
+             img_tvec=np.array([imgs[i].tvec for i in sorted(imgs)]),
+             pt_ids=np.array(sorted(pts)), pt_xyz=np.array([pts[i].xyz for i in sorted(pts)]),
+             pt_rgb=np.array([pts[i].rgb for i in sorted(pts)]))
+    np.savez_compressed(out / "ref_colmap_reader.npz", **d)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", required=True)
+    ap.add_argument("--sets", nargs="+", default=["fixtures", "comparisons", "densify", "colmap"],
+                    choices=["fixtures", "comparisons", "densify", "colmap"])
+    args = ap.parse_args()
+    out = Path(args.out)
+    out.mkdir(parents=True, exist_ok=True)
+    meta = dict(torch=torch.__version__)
+    if "colmap" in args.sets:
+        colmap(out, meta)
+    if set(args.sets) - {"colmap"}:
+        dev = torch.device("cuda")
+        ref_ext, _ = ref_loader.load_reference()
+        meta["gpu"] = torch.cuda.get_device_name(0)
+        if "fixtures" in args.sets:
+            fixtures(out, dev, ref_ext, meta)
+        if "comparisons" in args.sets:
+            comparisons(out, dev, meta)
+        if "densify" in args.sets:
+            densify(out, dev, meta)
 
     import json
 
